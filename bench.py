@@ -12,6 +12,7 @@ batch 16; `--config 5` = cat->dog with two improved-DDPM 256x256 U-Nets, 250-ste
     python bench.py --gpus 1 --steps K --warmup W [--config 2|4|5]      # our engine
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                                # the reference's CPU path (oracle port), rank 0 only
+    python bench.py ... --dump-outputs DIR                              # also save the last timed step's images as DIR/images.npy
 
 Prints ONE JSON line.  `value` is timed with inputs resident in HBM; `e2e` goes through the drop-in wrapper API with HOST
 buffers (H2D of image / conditioning / noise and D2H of the result inside the timed region).  `roofline` comes from a separate
@@ -33,6 +34,7 @@ if ROOT not in sys.path:
 
 if os.environ.get('NCCL_DEBUG', '').upper() == 'VERSION':     # NCCL prints its banner to stdout: keep stdout = the one JSON line
     os.environ['NCCL_DEBUG'] = 'WARN'
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 UNIT = 'images/s'
@@ -115,6 +117,7 @@ def encode_noise(sched, n_rec, shape, gen):
 
 
 def timed(eng, fn, steps, warmup, world, dist):
+    """-> (ms of the `steps` timed calls, launches they issued, what the last timed call returned)."""
     d = eng.device
     for _ in range(warmup):
         fn()
@@ -126,7 +129,7 @@ def timed(eng, fn, steps, warmup, world, dist):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        fn()
+        out = fn()
     e1.record()
     torch.cuda.synchronize()
     if world > 1:
@@ -134,7 +137,14 @@ def timed(eng, fn, steps, warmup, world, dist):
     ms = torch.tensor([e0.elapsed_time(e1)], device=d)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-    return float(ms.item()), eng.launches - l0
+    return float(ms.item()), eng.launches - l0, out
+
+
+def dump_outputs(path, **arrays):
+    """Each array -> path/<name>.npy (float32), so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a.detach().float().cpu().numpy())
 
 
 def time_call(fn, reps=3, warm=2):
@@ -307,6 +317,7 @@ def run_ours(args):
         src, tgt = nets
         psched = PixelSchedule('ddim', S, S, ETA, 999)
         n_rec = S - 1
+        # the first draw from the device's default generator, which starts from torch's fixed default seed: the same in every run
         noise_dev = torch.randn(n_rec + 1, B, 3, RES, RES, device=d)       # resident arm: noise lives in HBM (1.5 GB at B=8)
         last_dev = torch.zeros(1, B, 3, RES, RES, device=d)
         img_dev = image.to(d)
@@ -335,10 +346,13 @@ def run_ours(args):
 
     clocks = ClockSampler(local)
     clocks.start()
-    ms_total, launches = timed(eng, cycle_resident, args.steps, args.warmup, world, dist)
+    ms_total, launches, images = timed(eng, cycle_resident, args.steps, args.warmup, world, dist)
     clk = clocks.stop()
+    # rank 0's inputs are those of the single-GPU run, so its images are comparable across --gpus
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, images=images)
     e2e_steps = max(1, min(args.steps, 2))
-    ms_e2e, _ = timed(eng, cycle_e2e, e2e_steps, 1, world, dist)
+    ms_e2e, _, _ = timed(eng, cycle_e2e, e2e_steps, 1, world, dist)
     value = world * B * args.steps / (ms_total / 1e3)
     e2e_value = world * B * e2e_steps / (ms_e2e / 1e3)
 
@@ -547,12 +561,16 @@ def build_parser():
     ap.add_argument('--mma', type=int, default=None, help='0 FFMA fp32, 1 tcgen05 fp16-split (default), 3 tcgen05 3xTF32, 4 fast path')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-fast', action='store_true', help='skip the fast-path probe')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the images of the last timed step (rank 0's batch) to DIR/images.npy, float32")
     return ap
 
 
 if __name__ == '__main__':
     ap = build_parser()
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -302,6 +302,8 @@ def golden_pixel_cycle():
             print(f'pixel_cycle[{tag}]: 1-ulp sensitivity of the reference decode {float(out[f"sens_{tag}"]):.3e}')
             print(f'pixel_cycle[{tag}]: z {tuple(z.shape)} |z|max {z.abs().max():.2f}  recon max|img-image| '
                   f'{(img - image).abs().max():.3e}')
+        # the refinement acts on the decode only: its z is the 'ddim' encode, stored once (keeps the fixture under 1 MB)
+        assert torch.equal(out.pop('z_ddim_refine'), out['z_ddim'])
         save('pixel_cycle_iddpm64', **out)
     finally:
         os.chdir(cwd)

@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -16,7 +17,7 @@ def test_defaults_are_the_single_gpu_headline():
     import bench
     ap = bench.build_parser()
     a = ap.parse_args([])
-    assert a.gpus == 1 and a.config == 2 and a.warmup >= 3 and a.impl == 'ours'
+    assert a.gpus == 1 and a.config == 2 and a.warmup >= 3 and a.impl == 'ours' and a.dump_outputs is None
 
 
 def test_host_thread_budget_is_sane():
@@ -33,9 +34,11 @@ def test_bench_never_routes_the_product_through_the_oracle():
 
 
 @pytest.mark.gpu
-def test_live_bench_line_has_the_contract_keys():
-    """One short real run (LDM 256^2 configuration, 1 timed step, no CPU leg): every contract key, consistent bookkeeping."""
-    r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--config', '4', '--steps', '1', '--warmup', '3', '--no-cpu', '--no-fast'],
+def test_live_bench_line_has_the_contract_keys(tmp_path):
+    """One short real run (LDM 256^2 configuration, 1 timed step, no CPU leg): every contract key, consistent bookkeeping, and the
+    images of the timed step written by --dump-outputs."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--config', '4', '--steps', '1', '--warmup', '3', '--no-cpu', '--no-fast',
+                        '--dump-outputs', str(tmp_path)],
                        capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     d = json.loads(r.stdout.strip().splitlines()[-1])
@@ -54,3 +57,6 @@ def test_live_bench_line_has_the_contract_keys():
     assert d['e2e']['value'] < 1.1 * d['value']
     # the two loop drivers agree
     assert d['two_phase']['max_abs_diff_lockstep_vs_two_phase'] < 1e-3
+    assert sorted(os.listdir(tmp_path)) == ['images.npy']
+    img = np.load(tmp_path / 'images.npy')
+    assert img.dtype == np.float32 and img.shape == (d['config']['global_batch'], 3, 256, 256) and np.isfinite(img).all()

@@ -68,7 +68,7 @@ def test_pixel_wrapper_vs_reference_fixture(eng, tag, kw):
     assert (w.resolution, w.channels, w.latent_dim) == (64, 3, 64 * 64 * 3 * kw['es_steps'])
     torch.manual_seed(2000)
     z = w.encode(g['image'])
-    zref = g[f'z_{tag}']
+    zref = g['z_ddim' if tag == 'ddim_refine' else f'z_{tag}']       # the refinement acts on the decode only: same encode as 'ddim'
     rz = maxdiff(z.cpu(), zref) / float(zref.abs().max())
     # (the fixture's decode continues the encode's CPU RNG stream; our encode consumed the same number of draws)
     img = w(zref).cpu()
