@@ -42,6 +42,24 @@ class PixelCoef(C.Structure):
                 ('weight', C.c_float), ('inv_sqrt_1m_bt', C.c_float), ('std_model', C.c_float), ('mask', C.c_float)]
 
 
+class GemmPlan(C.Structure):
+    _fields_ = [('path', C.c_int), ('halo', C.c_int), ('epi_tma', C.c_int), ('tn_w', C.c_int), ('splits', C.c_int), ('tail16', C.c_int),
+                ('side_done', C.c_int)]
+
+
+GEMM_PATHS = {0: 'FFMA', 1: 'SS', 2: 'TS', 3: 'H16', 4: 'H16_PAIR'}
+
+
+class GemmTest(C.Structure):
+    _fields_ = [('conv', C.c_int), ('M', C.c_int), ('B', C.c_int), ('H', C.c_int), ('W', C.c_int), ('stride', C.c_int), ('pad', C.c_int),
+                ('up', C.c_int), ('N', C.c_int), ('C1', C.c_int), ('C2', C.c_int), ('A', C.c_void_p), ('A2', C.c_void_p),
+                ('a_amax', C.c_void_p), ('a2_amax', C.c_void_p), ('w', C.c_void_p), ('bias', C.c_void_p), ('rowvec', C.c_void_p),
+                ('ld_rowvec', C.c_int), ('rows_per_batch', C.c_int), ('residual', C.c_void_p), ('ldr', C.c_int), ('alpha', C.c_float),
+                ('geglu', C.c_int), ('C', C.c_void_p), ('ldc', C.c_int), ('out_nchw', C.c_int), ('rows_per_img', C.c_int),
+                ('C_lo', C.c_void_p), ('Ct_hi', C.c_void_p), ('Ct_lo', C.c_void_p), ('t_col0', C.c_int), ('ldt', C.c_longlong),
+                ('c_amax', C.c_void_p), ('c_stats', C.c_void_p), ('plan', C.POINTER(GemmPlan))]
+
+
 _P = C.c_void_p          # device / opaque pointers
 _F = C.c_float
 _I = C.c_int
@@ -99,9 +117,8 @@ SIGNATURES = {
     'cdx_image_metrics': (_I, [_P, _P, _P, _I, _I, _I, _P, _P]),
     'cdx_pixel_encode': (_I, [_P, _P, C.POINTER(PixelCoef), C.POINTER(_F), _I, _P, _F, _F, _P, _I, _I, _I, _P]),
     'cdx_pixel_decode': (_I, [_P, _P, _I, C.POINTER(PixelCoef), C.POINTER(_F), _I, _P, _P, _I, _I, _I, _P]),
-    'cdx_op_conv3x3': (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
-    'cdx_op_linear': (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P]),
-    'cdx_op_groupnorm': (_I, [_P, _P, _P, _P, _F, _I, _P, _I, _I, _I, _P]),
+    'cdx_op_gemm': (_I, [_P, C.POINTER(GemmTest), _P]),
+    'cdx_op_groupnorm': (_I, [_P, _P, _I, _P, _I, _P, _P, _F, _I, _P, _P, _I, _P, _P, _P, _P, _I, _I, _P]),
     'cdx_op_layernorm': (_I, [_P, _P, _P, _P, _P, _I, _I, _P]),
     'cdx_op_attention': (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P]),
     'cdx_op_nchw_to_nhwc': (_I, [_P, _P, _P, _I, _I, _I, _P]),

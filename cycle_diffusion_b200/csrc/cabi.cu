@@ -623,68 +623,95 @@ int cdx_pixel_decode(cdx_net* un, const float* z, int n_eps, const cdx_pixel_coe
 }
 
 // ---------------------------------------------------------------- unit-test hooks
-int cdx_op_conv3x3(cdx_engine* eh, const float* x, const float* w_oihw, const float* bias, float* y, int B, int H, int W, int Cin, int Cout,
-                   int stride, int pad_lo, int upsample, void* stream) {
+int cdx_op_gemm(cdx_engine* eh, const cdx_gemm_test* t, void* stream) {
   return guard([&] {
-    CDX_CHECK(eh && x && w_oihw && y, "op_conv3x3: null argument");
+    CDX_CHECK(eh && t && t->A && t->w && t->C && t->N > 0 && t->C1 > 0, "op_gemm: null argument / empty problem");
+    CDX_CHECK(!t->A2 || (!t->conv && t->C2 > 0), "op_gemm: a second source needs dense mode and C2 > 0");
+    CDX_CHECK(!t->geglu || (!t->conv && (t->N % 128) == 0 && !t->c_stats), "op_gemm: GEGLU needs dense mode, N %% 128 == 0 and no statistics");
     Engine& e = eh->e;
     cudaStream_t s = S(stream);
+    const int C2 = t->A2 ? t->C2 : 0;
+    GemmArgs g;
+    g.N = t->N;
+    if (t->conv) {
+      CDX_CHECK(t->B > 0 && t->H > 0 && t->W > 0 && (t->stride == 1 || t->stride == 2) && t->up >= 1, "op_gemm: bad conv geometry");
+      const int Hl = t->H * t->up, Wl = t->W * t->up;
+      g.mode = 1;
+      g.Hout = t->stride == 1 ? Hl : Hl / 2;
+      g.Wout = t->stride == 1 ? Wl : Wl / 2;
+      g.M = t->B * g.Hout * g.Wout; g.K = 9 * t->C1;
+      g.Hin = t->H; g.Win = t->W; g.stride = t->stride; g.pad = t->pad; g.up = t->up;
+    } else {
+      CDX_CHECK(t->M > 0, "op_gemm: M = %d", t->M);
+      g.M = t->M; g.K = t->C1 + C2;
+    }
+    const int rows_img = t->conv ? g.Hout * g.Wout : g.M;
+    g.A = t->A; g.lda = t->C1; g.C1 = t->C1;
+    g.A2 = t->A2; g.lda2 = C2; g.C2 = C2;
+    g.a_amax = t->a_amax; g.a2_amax = t->a2_amax;
+    g.ldb = g.K;
+    g.rowvec = t->rowvec; g.ld_rowvec = t->ld_rowvec;
+    g.rows_per_batch = t->rows_per_batch > 0 ? t->rows_per_batch : rows_img;
+    g.residual = t->residual; g.ldr = t->ldr > 0 ? t->ldr : t->N;
+    g.alpha = t->alpha;
+    g.geglu = t->geglu;
+    g.Cout = t->C; g.ldc = t->ldc > 0 ? t->ldc : (t->geglu ? t->N / 2 : t->N);
+    g.out_nchw = t->out_nchw; g.rows_per_img = t->rows_per_img > 0 ? t->rows_per_img : rows_img;
+    g.Cout_lo = t->C_lo;
+    g.Ct_hi = t->Ct_hi; g.Ct_lo = t->Ct_lo; g.t_col0 = t->t_col0; g.ldt = t->ldt > 0 ? t->ldt : g.M;
+    g.c_amax = t->c_amax; g.c_stats = t->c_stats;
+    CDX_CHECK(!t->c_stats || g.M % g.rows_per_batch == 0, "op_gemm: statistics need whole images (M=%d, rows_per_batch=%d)", g.M, g.rows_per_batch);
     with_arena(e, s, [&] {
       Scope sc(e.arena);
       e.pools_reset(s);
-      float* wr = (float*)e.arena.alloc((size_t)Cout * Cin * 9 * sizeof(float));
-      repack_conv3x3(e, w_oihw, wr, Cout, Cin, s);
-      const int Hl = H * upsample, Wl = W * upsample;
-      GemmArgs g;
-      g.mode = 1;
-      g.Hout = stride == 1 ? Hl : Hl / 2;
-      g.Wout = stride == 1 ? Wl : Wl / 2;
-      g.M = B * g.Hout * g.Wout; g.N = Cout; g.K = 9 * Cin;
-      g.A = x; g.lda = Cin; g.C1 = Cin;
-      g.Hin = H; g.Win = W; g.stride = stride; g.pad = pad_lo; g.up = upsample;
-      g.Bw = wr; g.ldb = 9 * Cin;
-      g.Cout = y; g.ldc = Cout;
-      g.bias = bias;
-      if (e.mma_mode == 1) {   // exercise the TS kernel: build the TF32 planes of the (repacked) weight on the fly
-        float* hi = (float*)e.arena.alloc((size_t)Cout * Cin * 9 * sizeof(float));
-        float* lo = (float*)e.arena.alloc((size_t)Cout * Cin * 9 * sizeof(float));
-        split_planes(e, wr, hi, lo, (size_t)Cout * Cin * 9, s);
+      e.last_gemm = cdx_gemm_plan{-1, 0, 0, 0, 0, 0, 0};
+      const size_t nw = (size_t)g.N * g.K;
+      // the weight as the networks store it: conv3x3 repacked O,kh,kw,I; GEGLU rows as [32 value | 32 gate] blocks (bias too)
+      const float* w = t->w;
+      if (t->conv) {
+        float* wr = (float*)e.arena.alloc(nw * sizeof(float));
+        repack_conv3x3(e, t->w, wr, g.N, t->C1, s);
+        w = wr;
+      } else if (t->geglu) {
+        float* wi = (float*)e.arena.alloc(nw * sizeof(float));
+        interleave_geglu_rows(e, t->w, wi, g.N, g.K, s);
+        w = wi;
+      }
+      g.Bw = w;
+      g.bias = t->bias;
+      if (t->geglu && t->bias) {
+        float* bi = (float*)e.arena.alloc((size_t)g.N * sizeof(float));
+        interleave_geglu_rows(e, t->bias, bi, g.N, 1, s);
+        g.bias = bi;
+      }
+      if (e.mma_mode == 1) {   // the operand planes the networks build at finalize: TF32 (TS kernel) and fp16-split
+        float* hi = (float*)e.arena.alloc(nw * sizeof(float));
+        float* lo = (float*)e.arena.alloc(nw * sizeof(float));
+        split_planes(e, w, hi, lo, nw, s);
         g.Bw_hi = hi; g.Bw_lo = lo;
-        hook_h16_planes(e, wr, (size_t)Cout * Cin * 9, g, s);
+        hook_h16_planes(e, w, nw, g, s);
+      }
+      if (!e.dry()) {
+        if (t->c_amax) CDX_CUDA(cudaMemsetAsync(t->c_amax, 0, sizeof(float), s));
+        if (t->c_stats) CDX_CUDA(cudaMemsetAsync(t->c_stats, 0, (size_t)(g.M / g.rows_per_batch) * g.N * 2 * sizeof(double), s));
       }
       gemm(e, g, s);
     });
+    if (t->plan) *t->plan = e.last_gemm;
   });
 }
-int cdx_op_linear(cdx_engine* eh, const float* x, const float* w, const float* bias, float* y, int M, int K, int N, void* stream) {
-  return guard([&] {
-    CDX_CHECK(eh && x && w && y, "op_linear: null argument");
-    Engine& e = eh->e;
-    with_arena(e, S(stream), [&] {
-      Scope sc(e.arena);
-      e.pools_reset(S(stream));
-      GemmArgs g;
-      g.M = M; g.N = N; g.K = K;
-      g.A = x; g.lda = K; g.C1 = K;
-      g.Bw = w; g.ldb = K;
-      g.Cout = y; g.ldc = N;
-      g.bias = bias;
-      if (e.mma_mode == 1) {
-        float* hi = (float*)e.arena.alloc((size_t)N * K * sizeof(float));
-        float* lo = (float*)e.arena.alloc((size_t)N * K * sizeof(float));
-        split_planes(e, w, hi, lo, (size_t)N * K, S(stream));
-        g.Bw_hi = hi; g.Bw_lo = lo;
-        hook_h16_planes(e, w, (size_t)N * K, g, S(stream));
-      }
-      gemm(e, g, S(stream));
-    });
-  });
-}
-int cdx_op_groupnorm(cdx_engine* eh, const float* x, const float* gamma, const float* beta, float eps, int silu_, float* y, int B, int HW, int C,
+int cdx_op_groupnorm(cdx_engine* eh, const float* x, int C1, const float* x2, int C2, const float* gamma, const float* beta, float eps, int silu_,
+                     const float* scale, const float* shift, int ld_ss, const double* st1, const double* st2, float* amax, float* y, int B, int HW,
                      void* stream) {
   return guard([&] {
-    CDX_CHECK(eh && x && gamma && beta && y, "op_groupnorm: null argument");
-    with_arena(eh->e, S(stream), [&] { eh->e.pools_reset(S(stream)); groupnorm(eh->e, x, C, nullptr, 0, gamma, beta, eps, silu_ != 0, nullptr, nullptr, 0, y, B, HW, S(stream)); });
+    CDX_CHECK(eh && x && gamma && beta && y && (!x2 || C2 > 0), "op_groupnorm: null argument");
+    Engine& e = eh->e;
+    cudaStream_t s = S(stream);
+    with_arena(e, s, [&] {
+      e.pools_reset(s);
+      if (amax && !e.dry()) CDX_CUDA(cudaMemsetAsync(amax, 0, sizeof(float), s));
+      groupnorm(e, x, C1, x2, x2 ? C2 : 0, gamma, beta, eps, silu_ != 0, scale, shift, ld_ss, y, B, HW, s, st1, st2, amax);
+    });
   });
 }
 int cdx_op_layernorm(cdx_engine* eh, const float* x, const float* gamma, const float* beta, float* y, int M, int C, void* stream) {

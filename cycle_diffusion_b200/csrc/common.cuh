@@ -90,6 +90,7 @@ struct Engine {
   cudaEvent_t done_ev = nullptr;
   bool ev_recorded = false;
   uint64_t launches = 0;
+  cdx_gemm_plan last_gemm{};      // variant taken by the most recent GEMM's real pass (host only; read by the op-level test hook)
   bool dry() const { return arena.dry; }
 };
 

@@ -355,6 +355,7 @@ void gemm(Engine& e, const GemmArgs& a, cudaStream_t s) {
     split_planes(e, a.Cout, a.Cout, a.Cout_lo, (size_t)a.M * a.N, s);
     return;
   }
+  e.last_gemm = cdx_gemm_plan{CDX_GEMM_FFMA, 0, 0, 0, 1, 0, 0};
   const double zz = (double)a.batch * a.heads;
   ProfScope ps(e, s, a.batch * a.heads > 1 ? PROF_BATCHED_FFMA : (a.mode == 1 ? PROF_CONV_FFMA : PROF_DENSE_FFMA),
                2.0 * a.M * a.N * a.K * zz, 4.0 * zz * ((double)a.M * a.K / (a.mode == 1 ? 9 : 1) + (double)a.N * a.K + (double)a.M * a.N), 1);

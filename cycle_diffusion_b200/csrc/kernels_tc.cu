@@ -800,7 +800,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
             const long long at = (long long)(n - p.t_col0) * p.ldt + m;
             p.Ct_hi[at] = hi;
             p.Ct_lo[at] = __uint_as_float(rn_tf32(__float_as_uint(o - hi)));
-            omax = fmaxf(omax, fabsf(o));
+            omax = fmaxf(omax, fabsf(hi));                        // the range of the stored hi plane, as for the row-major planes
           }
         }
       }
@@ -865,13 +865,17 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
             bulk_commit();
           }
           if (p.c_stats) {
-            // GroupNorm statistics of the tensor being written, from the staged block (the warp's 32 rows lie inside one image)
+            // GroupNorm statistics of the tensor being written, from the staged block (the warp's 32 rows lie inside one image).
+            // The fp32 partial sums are taken about the column's row-0 value v0 and re-centred in fp64: plain fp32 sums of x and
+            // x^2 lose the variance when |mean| >> std (E[x^2] - mean^2 cancels; |mean| / std = 100 costs 4e-5 of the normalised output)
             const float* const sf = reinterpret_cast<const float*>(stg);
+            const int col = NC == 8 ? lane : (lane & 15);
+            const float v0 = sf[(sidx(0, col >> 2) << 2) | (lane & 3)];
             float cs = 0.f, cq = 0.f;
             if (NC == 8) {                       // lane -> column, all 32 rows (the swizzle permutes chunks: no bank conflict)
 #pragma unroll
               for (int rr = 0; rr < 32; ++rr) {
-                const float v = sf[(sidx(rr, lane >> 2) << 2) | (lane & 3)];
+                const float v = sf[(sidx(rr, lane >> 2) << 2) | (lane & 3)] - v0;
                 cs += v; cq += v * v;
               }
             } else {                             // lane & 15 -> column, half-warp -> 16 rows (opposite row parity: different banks)
@@ -879,16 +883,17 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
 #pragma unroll
               for (int i = 0; i < 16; ++i) {
                 const int rr = hh * 16 + (i ^ hh);
-                const float v = sf[(sidx(rr, (lane & 15) >> 2) << 2) | (lane & 3)];
+                const float v = sf[(sidx(rr, (lane & 15) >> 2) << 2) | (lane & 3)] - v0;
                 cs += v; cq += v * v;
               }
               cs += __shfl_xor_sync(0xffffffffu, cs, 16);
               cq += __shfl_xor_sync(0xffffffffu, cq, 16);
             }
             if (NC == 8 || lane < 16) {
-              double* st = p.c_stats + ((long long)(trow0 / p.rows_per_batch) * p.N + (tcol0 + part * 32 + (NC == 8 ? lane : (lane & 15)))) * 2;
-              atomicAdd(st, (double)cs);
-              atomicAdd(st + 1, (double)cq);
+              double* st = p.c_stats + ((long long)(trow0 / p.rows_per_batch) * p.N + (tcol0 + part * 32 + col)) * 2;
+              const double s0 = v0, ds = cs;
+              atomicAdd(st, ds + 32.0 * s0);
+              atomicAdd(st + 1, (double)cq + s0 * (2.0 * ds + 32.0 * s0));
             }
           }
           if (p.C_lo) {
@@ -1008,14 +1013,22 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
           }
           if (p.c_stats) {
             // GroupNorm statistics of the tensor being written: this thread holds 4 columns x 4 rows here (8 rows over both
-            // halves); rows of one quadrant belong to one image
+            // halves); rows of one quadrant belong to one image.  Partial sums about the quadrant's row-0 values, re-centred in fp64
+            // below (see the TMA epilogue).  Lane g (rsub 0) is the only reader of row 0's staged chunk g: it puts the final row-0
+            // value there, where every lane finds it until the next block is staged (after the fold's shuffles below)
+            if (half == 0) {
+              if (rsub == 0) stg[g] = o[0];
+              __syncwarp();
+            }
+            const float4 v0 = stg[g];
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
               if (mm[half * 4 + i] >= 0) {
-                gs[0] += o[i].x; gq[0] += o[i].x * o[i].x;
-                gs[1] += o[i].y; gq[1] += o[i].y * o[i].y;
-                gs[2] += o[i].z; gq[2] += o[i].z * o[i].z;
-                gs[3] += o[i].w; gq[3] += o[i].w * o[i].w;
+                const float dx = o[i].x - v0.x, dy = o[i].y - v0.y, dz = o[i].z - v0.z, dw = o[i].w - v0.w;
+                gs[0] += dx; gq[0] += dx * dx;
+                gs[1] += dy; gq[1] += dy * dy;
+                gs[2] += dz; gq[2] += dz * dz;
+                gs[3] += dw; gq[3] += dw * dw;
               }
             }
           }
@@ -1038,6 +1051,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
           }
         }
         if (p.c_stats) {
+          const float4 v0 = stg[g];                            // (read before the shuffles: the next block may be staged after them)
           // fold the 4 row-subgroups (lanes g, g+8, g+16, g+24), then one fp64 atomic per (column, statistic)
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
@@ -1045,12 +1059,15 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
             gs[j] += __shfl_xor_sync(0xffffffffu, gs[j], 16); gq[j] += __shfl_xor_sync(0xffffffffu, gq[j], 16);
           }
           const int mq = __shfl_sync(0xffffffffu, m32, 0) >= 0 ? __shfl_sync(0xffffffffu, m32, 0) : -1;   // first row of the quadrant
+          const double nv = (double)__popc(__ballot_sync(0xffffffffu, m32 >= 0));      // rows of the quadrant inside the tensor
           if (rsub == 0 && mq >= 0 && n < nlim && fin) {
             double* st = p.c_stats + ((long long)(mq / p.rows_per_batch) * p.N + n) * 2;
+            const float v0a[4] = {v0.x, v0.y, v0.z, v0.w};
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
-              atomicAdd(st + 2 * j, (double)gs[j]);
-              atomicAdd(st + 2 * j + 1, (double)gq[j]);
+              const double s0 = v0a[j], ds = gs[j];
+              atomicAdd(st + 2 * j, ds + nv * s0);
+              atomicAdd(st + 2 * j + 1, (double)gq[j] + s0 * (2.0 * ds + nv * s0));
             }
           }
         }
@@ -1528,11 +1545,12 @@ bool gemm_tc(Engine& e, const GemmArgs& a, cudaStream_t s, int* side_done) {
   // TMA epilogue (TcParams::epi_tma): dense layers whose epilogue is the final one and needs no per-column statistics
   const CUtensorMap *mC = mA, *mClo = mA, *mR = mA, *mC16 = mA, *mClo16 = mA, *mR16 = mA;
   static const bool no_epi_tma = getenv("CDX_TC_NO_EPI_TMA") != nullptr;
+  bool tail16 = false;
   if (!no_epi_tma && h16 && a.mode == 0 && !a.out_nchw && p.splits == 1 && a.M >= TBM) {       // (compiled into the fp16-split kernels only)
     const uint64_t nc = (uint64_t)(a.geglu ? a.N / 2 : a.N);
     uint64_t d[2] = {nc, (uint64_t)a.M}, st[1] = {(uint64_t)a.ldc * 4};
     uint32_t bx[2] = {32, 32}, bx16[2] = {16, 32};
-    const bool tail16 = (p.tn_w & 31) != 0 || ((a.N % p.tn_w) & 31) != 0;      // some warp stores a 16-column tail slot
+    tail16 = (p.tn_w & 31) != 0 || ((a.N % p.tn_w) & 31) != 0;      // some warp stores a 16-column tail slot
     mC = &get_map(a.Cout, 2, d, st, bx);
     if (tail16) mC16 = &get_map(a.Cout, 2, d, st, bx16, nullptr, 4, 64);
     if (p.C_lo) {
@@ -1546,6 +1564,8 @@ bool gemm_tc(Engine& e, const GemmArgs& a, cudaStream_t s, int* side_done) {
     }
     p.epi_tma = 1;
   }
+  e.last_gemm = cdx_gemm_plan{h16 ? (cg2 ? CDX_GEMM_H16_PAIR : CDX_GEMM_H16) : ts ? CDX_GEMM_TS : CDX_GEMM_SS, p.halo, p.epi_tma, p.tn_w, p.splits,
+                              tail16 ? 1 : 0, (p.c_amax ? 1 : 0) | (p.c_stats ? 2 : 0)};
   ensure_attr(e.device);
   ProfScope ps(e, s, a.mode == 1 ? PROF_CONV_TC : PROF_DENSE_TC, 2.0 * a.M * a.N * a.K,
                4.0 * ((double)a.M * a.K / (a.mode == 1 ? 9 : 1) + (double)a.N * a.K + (double)a.M * a.N), 1);

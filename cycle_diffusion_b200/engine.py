@@ -157,24 +157,70 @@ class Engine:
 
     # ------------------------------------------------------------------ unit-test hooks (NHWC)
     def op_conv3x3(self, x_nhwc, w_oihw, bias, stride=1, pad_lo=1, upsample=1):
-        x, w = _f32c(x_nhwc, self.device), _f32c(w_oihw, self.device)
-        bias = _f32c(bias, self.device) if bias is not None else None
-        B, H, W, Cin = x.shape
-        Cout = w.shape[0]
-        Hl, Wl = H * upsample, W * upsample
-        Ho, Wo = (Hl, Wl) if stride == 1 else (Hl // 2, Wl // 2)
-        y = self.empty(B, Ho, Wo, Cout)
-        check(lib.cdx_op_conv3x3(self.h, _ptr(x), _ptr(w), _ptr(bias), _ptr(y), B, H, W, Cin, Cout, stride, pad_lo, upsample, self.stream))
-        return y
+        return self.op_gemm(x_nhwc, w_oihw, bias, conv=dict(stride=stride, pad=pad_lo, up=upsample))['C']
 
     def op_linear(self, x, w, bias):
-        x, w = _f32c(x, self.device), _f32c(w, self.device)
-        bias = _f32c(bias, self.device) if bias is not None else None
-        M, K = x.shape
+        return self.op_gemm(x, w, bias)['C']
+
+    def op_gemm(self, x, w, bias=None, *, conv=None, x2=None, a_amax=None, a2_amax=None, rowvec=None, rows_per_batch=0, residual=None,
+                alpha=1.0, geglu=False, out_nchw=False, planes=False, t_col0=None, c_amax=False, c_stats=False, ldc=0):
+        """One GEMM through cdx_op_gemm with the networks' epilogue options.
+
+        x: dense [M, C1] (x2: optional second source [M, C2]) or, with conv=dict(stride, pad, up), NHWC [B, H, W, C1] and w OIHW.
+        a_amax / a2_amax: optional one-element device tensors (tracked ranges).  geglu: w / bias in the reference [value; gate] layout.
+        planes: C and C_lo receive TF32 hi / lo planes; t_col0: columns >= t_col0 go transposed to Ct_hi / Ct_lo [N - t_col0, M]
+        (C then holds the first t_col0 columns, ldc = t_col0).  Returns a dict with C (and C_lo, Ct_hi, Ct_lo, c_amax, c_stats when
+        asked for) and `plan`, the variant that ran (_cabi.GemmPlan fields, path as a name)."""
+        dev = self.device
+        x, w = _f32c(x, dev), _f32c(w, dev)
+        opt = lambda t: _f32c(t, dev) if t is not None else None
+        bias, x2, rowvec, residual = opt(bias), opt(x2), opt(rowvec), opt(residual)
         N = w.shape[0]
-        y = self.empty(M, N)
-        check(lib.cdx_op_linear(self.h, _ptr(x), _ptr(w), _ptr(bias), _ptr(y), M, K, N, self.stream))
-        return y
+        t = _cabi.GemmTest()
+        if conv is not None:
+            B, H, W, C1 = x.shape
+            stride, pad, up = conv.get('stride', 1), conv.get('pad', 1), conv.get('up', 1)
+            Ho, Wo = (H * up, W * up) if stride == 1 else (H * up // 2, W * up // 2)
+            M, lead = B * Ho * Wo, (B, Ho, Wo)
+            t.conv, t.B, t.H, t.W, t.stride, t.pad, t.up = 1, B, H, W, stride, pad, up
+        else:
+            M, C1 = x.shape
+            lead = (M,)
+            t.M = M
+        ncols = N // 2 if geglu else (t_col0 if t_col0 is not None else N)
+        imgs = lead[0] if conv is not None else 1               # images (rows_per_batch default: one image per conv sample)
+        rpb = rows_per_batch or M // imgs
+        out = {'C': self.empty(imgs, N, M // imgs) if out_nchw else self.empty(*lead, ldc or ncols)}
+        t.N, t.C1 = N, C1
+        t.A, t.w, t.bias = _ptr(x), _ptr(w), _ptr(bias)
+        if x2 is not None:
+            t.A2, t.C2 = _ptr(x2), x2.shape[-1]
+        t.a_amax, t.a2_amax = _ptr(a_amax), _ptr(a2_amax)
+        if rowvec is not None:
+            t.rowvec, t.ld_rowvec = _ptr(rowvec), rowvec.shape[-1]
+        t.rows_per_batch = rpb
+        if residual is not None:
+            t.residual, t.ldr = _ptr(residual), residual.shape[-1]
+        t.alpha, t.geglu, t.out_nchw = float(alpha), int(geglu), int(out_nchw)
+        t.C, t.ldc = _ptr(out['C']), ldc or (0 if t_col0 is None else t_col0)
+        if planes:
+            out['C_lo'] = torch.empty_like(out['C'])
+            t.C_lo = _ptr(out['C_lo'])
+        if t_col0 is not None:
+            out['Ct_hi'], out['Ct_lo'] = self.empty(N - t_col0, M), self.empty(N - t_col0, M)
+            t.Ct_hi, t.Ct_lo, t.t_col0, t.ldt = _ptr(out['Ct_hi']), _ptr(out['Ct_lo']), t_col0, M
+        if c_amax:
+            out['c_amax'] = self.empty(1)
+            t.c_amax = _ptr(out['c_amax'])
+        if c_stats:
+            out['c_stats'] = torch.empty(M // rpb, N, 2, dtype=torch.float64, device=dev)
+            t.c_stats = _ptr(out['c_stats'])
+        plan = _cabi.GemmPlan()
+        t.plan = C.pointer(plan)
+        check(lib.cdx_op_gemm(self.h, C.byref(t), self.stream))
+        out['plan'] = {f: getattr(plan, f) for f, _ in _cabi.GemmPlan._fields_}
+        out['plan']['path'] = _cabi.GEMM_PATHS.get(plan.path, plan.path)
+        return out
 
     # ---- Directional-CLIP ranking / evaluation metrics (SURVEY 8f-3)
     def clip_preprocess(self, img, size=224):
@@ -202,12 +248,21 @@ class Engine:
         check(lib.cdx_image_metrics(self.h, _ptr(a), _ptr(b), B, H, W, _ptr(out), self.stream))
         return out
 
-    def op_groupnorm(self, x_nhwc, gamma, beta, eps, silu):
+    def op_groupnorm(self, x_nhwc, gamma, beta, eps, silu, x2=None, scale_shift=None, st1=None, st2=None, amax=False):
+        """GroupNorm(32) of x (or of the channel concat [x | x2]) -> [silu](gn * (1 + scale) + shift).  scale_shift: optional
+        [B, 2C] rows (scale first, as the improved-DDPM ResBlock chunks its embedding); st1 / st2: optional fp64 [B, C, 2] channel
+        statistics of the sources; amax=True returns (y, max |y| as a one-element tensor)."""
         x, gamma, beta = (_f32c(t, self.device) for t in (x_nhwc, gamma, beta))
-        B, H, W, Cc = x.shape
-        y = torch.empty_like(x)
-        check(lib.cdx_op_groupnorm(self.h, _ptr(x), _ptr(gamma), _ptr(beta), eps, int(silu), _ptr(y), B, H * W, Cc, self.stream))
-        return y
+        x2, ss = (_f32c(t, self.device) if t is not None else None for t in (x2, scale_shift))
+        st1, st2 = (t.to(self.device).contiguous() if t is not None else None for t in (st1, st2))
+        B, H, W, C1 = x.shape
+        C2 = x2.shape[-1] if x2 is not None else 0
+        y = self.empty(B, H, W, C1 + C2)
+        am = self.empty(1) if amax else None
+        scale, shift, ld_ss = (ss, ss[:, C1 + C2:], ss.shape[-1]) if ss is not None else (None, None, 0)
+        check(lib.cdx_op_groupnorm(self.h, _ptr(x), C1, _ptr(x2), C2, _ptr(gamma), _ptr(beta), eps, int(silu), _ptr(scale), _ptr(shift), ld_ss,
+                                   _ptr(st1), _ptr(st2), _ptr(am), _ptr(y), B, H * W, self.stream))
+        return (y, am) if amax else y
 
     def op_layernorm(self, x, gamma, beta):
         x, gamma, beta = (_f32c(t, self.device) for t in (x, gamma, beta))

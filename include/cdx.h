@@ -312,14 +312,64 @@ int cdx_pixel_decode(cdx_net* unet, const float* z, int n_eps, const cdx_pixel_c
                      int C, int R, void* stream);
 
 /* ---------------------------------------------------------------- unit-test hooks ----------- */
-/* Individual ops exported for per-op parity tests (tests/test_ops_gpu.py).  NHWC = [B,H,W,C]. */
-int cdx_op_conv3x3(cdx_engine* e, const float* x_nhwc, const float* w_oihw, const float* bias,
-                   float* y_nhwc, int B, int H, int W, int Cin, int Cout, int stride, int pad_lo,
-                   int upsample, void* stream);
-int cdx_op_linear(cdx_engine* e, const float* x, const float* w, const float* bias, float* y, int M,
-                  int K, int N, void* stream);
-int cdx_op_groupnorm(cdx_engine* e, const float* x_nhwc, const float* gamma, const float* beta,
-                     float eps, int silu, float* y_nhwc, int B, int HW, int C, void* stream);
+/* Individual ops exported for per-op parity tests (tests/test_ops_gpu.py, tests/test_gemm_epilogue_gpu.py).
+ * NHWC = [B,H,W,C].  Not part of the drop-in interface: these may change without an ABI version bump. */
+
+/* Which GEMM variant ran (filled on the real pass of the call, host side only). */
+#define CDX_GEMM_FFMA 0      /* SIMT fp32 tiles */
+#define CDX_GEMM_SS 1        /* tcgen05 3 x kind::tf32, both operands split in the kernel */
+#define CDX_GEMM_TS 2        /* tcgen05 3 x kind::tf32 on pre-split weight planes */
+#define CDX_GEMM_H16 3       /* tcgen05 3 x kind::f16 fp16-split, single CTA */
+#define CDX_GEMM_H16_PAIR 4  /* the same on CTA pairs (cta_group::2) */
+typedef struct cdx_gemm_plan {
+  int path;          /* CDX_GEMM_* */
+  int halo;          /* conv3x3 halo schedule */
+  int epi_tma;       /* TMA-store epilogue (else the per-row epilogue, or split-K partials + reduce kernel) */
+  int tn_w;          /* tile width along N */
+  int splits;        /* split-K factor (> 1: partial sums reduced by a second kernel) */
+  int tail16;        /* the TMA epilogue stores some 16-column tail boxes */
+  int side_done;     /* bit 0: c_amax produced by the GEMM kernels, bit 1: c_stats produced by the epilogue (else by an extra pass) */
+} cdx_gemm_plan;
+
+/* One GEMM with the epilogue options the networks use:
+ *   C = alpha * A . W^T (+ bias[n]) (+ rowvec[m / rows_per_batch, n]) (+ residual[m, n])
+ * conv = 0: A [M, C1] (optionally | A2 [M, C2], a channel concat), W [N, C1 + C2].
+ * conv = 1: A is the implicit im2col of a 3x3 convolution over NHWC x [B, H, W, C1] (stride 1 / 2, `pad` zero rows / columns
+ *   before the image -- stride 2 with pad 0 is the VAE's (0,1,0,1) padding -- and nearest `up` x upsampling of the input);
+ *   W is OIHW [N, C1, 3, 3]; M = B * Ho * Wo.
+ * a_amax / a2_amax: optional device scalars >= max |A| / |A2| (as tracked by a producer); measured by the GEMM when null.
+ * geglu: W (and bias) in the reference layout [N/2 value rows; N/2 gate rows]; C [M, N/2] = value * gelu(gate).
+ * out_nchw: C stored as [M / rows_per_img, N, rows_per_img].  C_lo: C and C_lo receive the TF32 hi / lo planes of the result.
+ * Ct_hi / Ct_lo: columns n >= t_col0 stored transposed as TF32 planes at [(n - t_col0) * ldt + m].
+ * c_amax (float) / c_stats (double [M / rows_per_batch, N, 2]): optional device outputs, zeroed here, receive max |stored C| and the
+ * per-(image, channel) {sum, sum of squares} of C.  Zero ld* / rows_per_* fields take the dense defaults.
+ * plan: optional host output. */
+typedef struct cdx_gemm_test {
+  int conv;
+  int M;                                  /* dense */
+  int B, H, W, stride, pad, up;           /* conv */
+  int N, C1, C2;
+  const float* A; const float* A2;
+  const float* a_amax; const float* a2_amax;
+  const float* w; const float* bias;
+  const float* rowvec; int ld_rowvec; int rows_per_batch;
+  const float* residual; int ldr;
+  float alpha;
+  int geglu;
+  float* C; int ldc;
+  int out_nchw, rows_per_img;
+  float* C_lo;
+  float* Ct_hi; float* Ct_lo; int t_col0; long long ldt;
+  float* c_amax; double* c_stats;
+  cdx_gemm_plan* plan;
+} cdx_gemm_test;
+int cdx_op_gemm(cdx_engine* e, const cdx_gemm_test* t, void* stream);
+/* GroupNorm(32) of x [B,HW,C1] (optionally channel-concatenated with x2 [B,HW,C2]), y = [silu](gn(x) * (1 + scale) + shift) with
+ * scale / shift [B, *] rows of stride ld_ss (may be null).  st1 / st2: optional per-(image, channel) {sum, sum of squares} of x / x2
+ * (fp64, as a GEMM epilogue produces them), computed here when null.  amax: optional device scalar, receives max |y| (zeroed here). */
+int cdx_op_groupnorm(cdx_engine* e, const float* x_nhwc, int C1, const float* x2_nhwc, int C2, const float* gamma,
+                     const float* beta, float eps, int silu, const float* scale, const float* shift, int ld_ss,
+                     const double* st1, const double* st2, float* amax, float* y_nhwc, int B, int HW, void* stream);
 int cdx_op_layernorm(cdx_engine* e, const float* x, const float* gamma, const float* beta, float* y,
                      int M, int C, void* stream);
 /* softmax(q k^T * scale) v with q [B,Nq,heads*d], k/v [B,Nk,heads*d] -> [B,Nq,heads*d] */
