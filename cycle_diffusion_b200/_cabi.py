@@ -108,6 +108,8 @@ SIGNATURES = {
                                _P]),
     'cdx_cycle_lockstep': (_I, [_P, _P, _P, _P, _P, _I, _F, _F, C.POINTER(DdimCoef), C.POINTER(_F), _I, _P, _F, _F, _P, _P, _I, _I, _I, _I,
                                 _P]),
+    'cdx_cycle_lockstep_pair': (_I, [_P, _P, _P, _P, _P, _P, _I, _F, _F, C.POINTER(DdimCoef), C.POINTER(_F), _I, _P, _F, _F, _P, _P, _I, _I,
+                                     _I, _I, _P]),
     'cdx_latent_loop_ens': (_I, [_P, _I, _P, _P, _P, _P, _I, _P, _P, C.POINTER(DdimCoef), C.POINTER(_F), _I, _I, _P, _F, _F, _P, _I, _P, _P, _P,
                                  _I, _I, _I, _I, _P]),
     'cdx_clip_preprocess': (_I, [_P, _P, _I, _I, _I, _P, _P]),
@@ -117,6 +119,7 @@ SIGNATURES = {
     'cdx_image_metrics': (_I, [_P, _P, _P, _I, _I, _I, _P, _P]),
     'cdx_pixel_encode': (_I, [_P, _P, C.POINTER(PixelCoef), C.POINTER(_F), _I, _P, _F, _F, _P, _I, _I, _I, _P]),
     'cdx_pixel_decode': (_I, [_P, _P, _I, C.POINTER(PixelCoef), C.POINTER(_F), _I, _P, _P, _I, _I, _I, _P]),
+    'cdx_pixel_cycle_lockstep': (_I, [_P, _P, _P, C.POINTER(PixelCoef), C.POINTER(_F), _I, _P, _F, _F, _P, _P, _P, _I, _I, _I, _P]),
     'cdx_op_gemm': (_I, [_P, C.POINTER(GemmTest), _P]),
     'cdx_op_groupnorm': (_I, [_P, _P, _I, _P, _I, _P, _P, _F, _I, _P, _P, _I, _P, _P, _P, _P, _I, _I, _P]),
     'cdx_op_layernorm': (_I, [_P, _P, _P, _P, _P, _I, _I, _P]),

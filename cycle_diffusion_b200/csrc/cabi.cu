@@ -35,26 +35,38 @@ int guard(F&& f) {
 // The arena, the context K/V cache and the weight planes are reused from call to call with no synchronisation of their own,
 // which is only safe in stream order.  A caller that switches streams between calls is handed over explicitly: every call
 // records an event at its end, and a call arriving on a different stream first waits for it.
+// `e2` (optional): a second engine whose networks `f` also runs (the two-model loops); both arenas are sized by the same sizing
+// pass and both engines' hand-over events are honoured.
 template <class F>
-void with_arena(Engine& e, cudaStream_t s, F&& f) {
+void with_arenas(Engine& e, Engine* e2, cudaStream_t s, F&& f) {
+  Engine* es[2] = {&e, (e2 && e2 != &e) ? e2 : nullptr};
+  const int ne = es[1] ? 2 : 1;
+  if (es[1]) CDX_CHECK(es[1]->device == e.device, "two engines on different devices (%d, %d)", e.device, es[1]->device);
   CDX_CUDA(cudaSetDevice(e.device));
-  e.arena.begin_dry();
+  for (int k = 0; k < ne; ++k) es[k]->arena.begin_dry();
   try {
     f();
   } catch (...) {
-    e.arena.dry = false;
-    e.arena.off = 0;
+    for (int k = 0; k < ne; ++k) { es[k]->arena.dry = false; es[k]->arena.off = 0; }
     throw;
   }
-  e.arena.end_dry();
-  if (!e.done_ev) CDX_CUDA(cudaEventCreateWithFlags(&e.done_ev, cudaEventDisableTiming));
-  if (e.ev_recorded && e.last_stream != s) CDX_CUDA(cudaStreamWaitEvent(s, e.done_ev, 0));
+  for (int k = 0; k < ne; ++k) {
+    Engine& x = *es[k];
+    x.arena.end_dry();
+    if (!x.done_ev) CDX_CUDA(cudaEventCreateWithFlags(&x.done_ev, cudaEventDisableTiming));
+    if (x.ev_recorded && x.last_stream != s) CDX_CUDA(cudaStreamWaitEvent(s, x.done_ev, 0));
+  }
   f();
-  e.arena.off = 0;
-  CDX_CUDA(cudaEventRecord(e.done_ev, s));
-  e.ev_recorded = true;
-  e.last_stream = s;
+  for (int k = 0; k < ne; ++k) {
+    Engine& x = *es[k];
+    x.arena.off = 0;
+    CDX_CUDA(cudaEventRecord(x.done_ev, s));
+    x.ev_recorded = true;
+    x.last_stream = s;
+  }
 }
+template <class F>
+void with_arena(Engine& e, cudaStream_t s, F&& f) { with_arenas(e, nullptr, s, f); }
 
 inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
@@ -107,6 +119,9 @@ void hook_h16_planes(Engine& e, const float* w, size_t n, GemmArgs& g, cudaStrea
 // consumed by the target chain in registers, so no z buffer is needed -- the Diffusers CycleDiffusionPipeline loop shape).
 // Per step: one U-Net call on the batch [src segments | tgt segments] (a chain contributes [uncond, cond] when it runs with
 // classifier-free guidance, ddim.py:550-559, else one segment) and ONE fused elementwise launch (latent_step).
+// With a target network `tgt` (two-model lock-step, latentdiff_stochastic_wrapper.py:253-311 run as one loop) the source segments
+// go through `unet` and the target segments through `tgt`: two U-Net calls on the same contiguous xin / eout slices, each chain at
+// the batch it has in the two-phase loops.
 // ---------------------------------------------------------------------------------------------------------------------
 enum { LOOP_ENC = 1, LOOP_DEC = 2, LOOP_LOCK = 3 };
 struct LatentLoopArgs {
@@ -123,7 +138,7 @@ struct LatentLoopArgs {
   int B = 0, C = 0, h = 0, w = 0;
 };
 
-void run_latent_loop(Net& unet, const LatentLoopArgs& a, cudaStream_t s) {
+void run_latent_loop(Net& unet, const LatentLoopArgs& a, cudaStream_t s, Net* tgt = nullptr) {
   Engine& e = *unet.eng;
   const int B = a.B, chw = a.C * a.h * a.w;
   const size_t n = (size_t)B * chw;
@@ -138,6 +153,8 @@ void run_latent_loop(Net& unet, const LatentLoopArgs& a, cudaStream_t s) {
   Scope sc(e.arena);
   unet.ctxkv.valid = false;                    // the conditioning is fixed for this loop: its K / V are computed by the first step only
   struct Invalidate { Net& u; ~Invalidate() { u.ctxkv.valid = false; } } inval{unet};
+  if (tgt) tgt->ctxkv.valid = false;
+  struct InvalidateTgt { Net* u; ~InvalidateTgt() { if (u) u->ctxkv.valid = false; } } inval_tgt{tgt};
   float* xin = (float*)e.arena.alloc((size_t)nseg * n * sizeof(float));
   float* eout = (float*)e.arena.alloc((size_t)nseg * n * sizeof(float));
   float* ctx_in = (float*)e.arena.alloc((size_t)nseg * ctx_n * sizeof(float));
@@ -184,7 +201,14 @@ void run_latent_loop(Net& unet, const LatentLoopArgs& a, cudaStream_t s) {
   }
   const int iters = e.dry() ? std::min(loop_steps, 1) : loop_steps;
   for (int i = 0; i < iters; ++i) {
-    unet_forward(unet, xin, tdev + (size_t)i * nb, ctx_in, a.L, eout, nb, a.h, a.w, s, true);
+    if (!tgt) {
+      unet_forward(unet, xin, tdev + (size_t)i * nb, ctx_in, a.L, eout, nb, a.h, a.w, s, true);
+    } else {
+      const size_t ns = (size_t)nseg_src * B;
+      unet_forward(unet, xin, tdev + (size_t)i * nb, ctx_in, a.L, eout, (int)ns, a.h, a.w, s, true);
+      unet_forward(*tgt, xin + ns * chw, tdev + (size_t)i * nb + ns, ctx_in + (size_t)nseg_src * ctx_n, a.L, eout + ns * chw,
+                   nseg_tgt * B, a.h, a.w, s, true);
+    }
     LatentStep st;
     st.n = n; st.chw = chw;
     if (enc) {
@@ -523,6 +547,25 @@ int cdx_cycle_lockstep(cdx_net* un, const float* x0, const float* c_src, const f
   });
 }
 
+int cdx_cycle_lockstep_pair(cdx_net* src, cdx_net* tgt, const float* x0, const float* c_src, const float* c_tgt, const float* uc, int L,
+                            float src_scale, float tgt_scale, const cdx_ddim_coef* coef, const float* t_host, int n_steps, const float* noise,
+                            float sqrt_a_T, float sqrt_1ma_T, float* x_out, float* z_out, int B, int C, int h, int w, void* stream) {
+  return guard([&] {
+    CDX_CHECK(src && src->owner && tgt && tgt->owner && x0 && ((c_src && c_tgt) || L == 0) && coef && t_host && noise && x_out,
+              "cycle_lockstep_pair: null argument");
+    CDX_CHECK(n_steps >= 1 && B > 0, "cycle_lockstep_pair: n_steps=%d B=%d", n_steps, B);
+    CDX_CHECK(src->n->ucfg.context_dim == tgt->n->ucfg.context_dim, "cycle_lockstep_pair: context widths differ (%d, %d)",
+              src->n->ucfg.context_dim, tgt->n->ucfg.context_dim);
+    for (int i = 0; i < n_steps; ++i) CDX_CHECK(coef[i].sigma > 0.f, "cycle_lockstep_pair: eta must be > 0 (sigma[%d] == 0), ddim.py:268", i);
+    LatentLoopArgs a;
+    a.mode = LOOP_LOCK;
+    a.x0 = x0; a.c_src = c_src; a.c_tgt = c_tgt; a.uc = uc; a.L = L; a.s_scale = src_scale; a.t_scale = tgt_scale;
+    a.coef = coef; a.t_host = t_host; a.n_steps = n_steps; a.n_rec = n_steps; a.noise = noise; a.sa = sqrt_a_T; a.s1 = sqrt_1ma_T;
+    a.z_out = z_out; a.x_out = x_out; a.B = B; a.C = C; a.h = h; a.w = w;
+    with_arenas(src->owner->e, &tgt->owner->e, S(stream), [&] { run_latent_loop(*src->n, a, S(stream), tgt->n); });
+  });
+}
+
 int cdx_latent_loop_ens(cdx_net* un, int mode, const float* x0, const float* c_src, const float* c_tgt, const float* uc, int L,
                         const float* src_scales, const float* tgt_scales, const cdx_ddim_coef* coef, const float* t_host, int n_steps, int n_rec,
                         const float* noise, float sqrt_a_T, float sqrt_1ma_T, const float* z_in, int n_eps, const float* extra_noise,
@@ -618,6 +661,59 @@ int cdx_pixel_decode(cdx_net* un, const float* z, int n_eps, const cdx_pixel_coe
         pixel_step_with_eps(e, xa, et, nz, coef[i], dst, B, chw, net_chw, s);
         std::swap(xa, xb);
       }
+    });
+  });
+}
+
+int cdx_pixel_cycle_lockstep(cdx_net* src, cdx_net* tgt, const float* x0, const cdx_pixel_coef* coef, const float* t_host, int n_steps,
+                             const float* noise, float sqrt_a_T, float sqrt_1ma_T, const float* last_noise, float* x_out, float* z_out, int B,
+                             int C, int R, void* stream) {
+  return guard([&] {
+    CDX_CHECK(src && src->owner && tgt && tgt->owner && x0 && coef && t_host && noise && x_out, "pixel_cycle_lockstep: null argument");
+    CDX_CHECK(n_steps >= 1 && B > 0, "pixel_cycle_lockstep: n_steps=%d B=%d", n_steps, B);
+    Engine& e = src->owner->e;
+    Net& su = *src->n;
+    Net& tu = *tgt->n;
+    CDX_CHECK(su.ucfg.out_channels >= C && tu.ucfg.out_channels >= C, "pixel_cycle_lockstep: U-Nets with %d / %d output channels for C=%d",
+              su.ucfg.out_channels, tu.ucfg.out_channels, C);
+    cudaStream_t s = S(stream);
+    const int chw = C * R * R;
+    const int net_chw_s = su.ucfg.out_channels * R * R, net_chw_t = tu.ucfg.out_channels * R * R;
+    const size_t n = (size_t)B * chw;
+    const int n_rec = n_steps - 1;
+    with_arenas(e, &tgt->owner->e, s, [&] {
+      Scope sc(e.arena);
+      float* xa = (float*)e.arena.alloc(n * sizeof(float));
+      float* xb = (float*)e.arena.alloc(n * sizeof(float));
+      float* ya = (float*)e.arena.alloc(n * sizeof(float));
+      float* yb = (float*)e.arena.alloc(n * sizeof(float));
+      float* es = (float*)e.arena.alloc((size_t)B * net_chw_s * sizeof(float));
+      float* et = (float*)e.arena.alloc((size_t)B * net_chw_t * sizeof(float));
+      float* tdev = (float*)e.arena.alloc((size_t)n_steps * B * sizeof(float));
+      upload_timesteps(e, t_host, n_steps, B, tdev, s);
+      q_sample(e, x0, noise, sqrt_a_T, sqrt_1ma_T, xa, n, s);                          // sample_xt, DW:310-314 (incl. the DW:483 index quirk)
+      if (z_out) scatter_slot(e, xa, z_out, B, chw, n_steps, 0, s);
+      const float* y = xa;                                                           // the target chain starts from the same x_T
+      float* yn = ya;
+      const int iters = e.dry() ? std::min(n_rec, 1) : n_rec;
+      for (int i = 0; i < iters; ++i) {
+        unet_forward(su, xa, tdev + (size_t)i * B, nullptr, 0, es, B, R, R, s);
+        unet_forward(tu, y, tdev + (size_t)i * B, nullptr, 0, et, B, R, R, s);
+        PixelLockStep st;
+        st.n = n; st.chw = chw;
+        st.cs = coef[i]; st.ct = coef[i];
+        st.x0 = x0; st.xt = xa; st.noise = noise + (size_t)(1 + i) * n; st.x_next = xb;
+        st.et_src = es; st.net_chw_src = net_chw_s;
+        st.y = y; st.et_tgt = et; st.net_chw_tgt = net_chw_t; st.y_next = yn;
+        if (z_out) { st.z_out = z_out + (size_t)(1 + i) * chw; st.z_stride = (long long)n_steps * chw; }
+        pixel_lock_step(e, st, s);
+        std::swap(xa, xb);
+        y = yn;
+        yn = (yn == ya) ? yb : ya;
+      }
+      // the last target step (0, -1) has no recovered noise: its draw is multiplied by 0 (DU:115,131)
+      unet_forward(tu, y, tdev + (size_t)n_rec * B, nullptr, 0, et, B, R, R, s);
+      pixel_step_with_eps(e, y, et, last_noise, coef[n_rec], x_out, B, chw, net_chw_t, s);
     });
   });
 }

@@ -295,6 +295,19 @@ void pixel_compute_eps(Engine& e, const float* xt, const float* xt_next, const f
                        int B, int chw, int net_chw, cudaStream_t s);
 void pixel_step_with_eps(Engine& e, const float* xt, const float* et, const float* eps, const cdx_pixel_coef& c, float* out,
                          int B, int chw, int net_chw, cudaStream_t s);
+// One iteration of the two-model pixel cycle in one launch: x_next = sample_xt_next(x0, xt, noise) and
+// eps = compute_eps(xt, x_next, et_src) under cs (source chain), y_next = denoising_step_with_eps(y, et_tgt, eps) under ct (target
+// chain).  Same per-element arithmetic as the three kernels above.  U-Net outputs are [B, Cnet, H, W] of which the first C channels
+// are used (learn_sigma split, DW:236-238): net_chw_* = Cnet * H * W of each chain's network.
+struct PixelLockStep {
+  size_t n = 0; int chw = 0;                 // B*chw elements
+  cdx_pixel_coef cs{}, ct{};
+  const float* x0 = nullptr; const float* xt = nullptr; const float* noise = nullptr; float* x_next = nullptr;
+  const float* et_src = nullptr; int net_chw_src = 0;
+  const float* y = nullptr; const float* et_tgt = nullptr; int net_chw_tgt = 0; float* y_next = nullptr;
+  float* z_out = nullptr; long long z_stride = 0;   // optional: eps -> z_out[b*z_stride + r]
+};
+void pixel_lock_step(Engine& e, const PixelLockStep& a, cudaStream_t s);
 
 inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 

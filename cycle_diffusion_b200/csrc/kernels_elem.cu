@@ -6,6 +6,7 @@
 //   ddim_compute_eps        CFG combine + compute_eps tail      ddim.py:555-559, 575-579
 //   ddim_step_with_eps      CFG combine + p_sample_ddim_with_eps tail   ddim.py:613-617, 634-645
 //   pixel_*                 sample_xt_next / compute_eps / denoising_step_with_eps   ddpm_ddim_wrapper.py:114-307
+//   pixel_lock_step         the three above for a source and a target chain in one launch (two-model lock-step cycle)
 //   vae_posterior           DiagonalGaussianDistribution.sample * scale_factor      distributions.py:24-37, ddpm.py:536-543
 // Each is one launch instead of the reference's ~8-10 elementwise launches per step (SURVEY.md 2.2).
 #include "common.cuh"
@@ -287,31 +288,43 @@ __global__ void latent_init_kernel(const LatentInit a) {
   }
 }
 
+// Per-element arithmetic of the pixel samplers.  The single-purpose kernels below and the fused two-chain kernel call the same
+// functions, so a value computed by the lock-step loop is the value the two-phase loops compute, bit for bit.
+__device__ __forceinline__ float pixel_posterior_f(float x0, float xt, float nz, const cdx_pixel_coef& c) {
+  if (c.ddpm) {
+    const float mean = ADD(MUL(c.w0, x0), MUL(c.wt, xt));                                   // DW:293
+    return ADD(mean, MUL(c.post_std, nz));                                                  // DW:297
+  }
+  const float et = DIV(SUB(xt, MUL(c.sqrt_at, x0)), c.sqrt_1m_at);                          // DW:299
+  return ADD(ADD(MUL(c.sqrt_at_next, x0), MUL(c.c2, et)), MUL(c.c1, nz));                   // DW:302
+}
+__device__ __forceinline__ float pixel_eps_f(float xt, float xn, float et, const cdx_pixel_coef& c) {
+  if (c.ddpm) {
+    const float mean = MUL(c.inv_sqrt_1m_bt, SUB(xt, MUL(c.weight, et)));                   // DW:266
+    return DIV(SUB(xn, mean), c.std_model);                                                 // DW:268
+  }
+  const float x0_t = DIV(SUB(xt, MUL(et, c.sqrt_1m_at)), c.sqrt_at);                        // DW:271
+  return DIV(SUB(SUB(xn, MUL(c.sqrt_at_next, x0_t)), MUL(c.c2, et)), c.c1);                 // DW:275
+}
+__device__ __forceinline__ float pixel_step_f(float xt, float et, float nz, const cdx_pixel_coef& c) {
+  if (c.ddpm) {
+    const float mean = MUL(c.inv_sqrt_1m_bt, SUB(xt, MUL(c.weight, et)));                   // DW:204
+    return ADD(mean, MUL(MUL(c.mask, c.std_model), nz));                                    // DW:208
+  }
+  const float x0_t = DIV(SUB(xt, MUL(et, c.sqrt_1m_at)), c.sqrt_at);                        // DW:213
+  return ADD(ADD(MUL(c.sqrt_at_next, x0_t), MUL(c.c2, et)), MUL(c.c1, nz));                 // DW:222
+}
+
 __global__ void pixel_posterior_kernel(const float* __restrict__ x0, const float* __restrict__ xt, const float* __restrict__ nz,
                                        cdx_pixel_coef c, float* __restrict__ out, size_t n) {
-  GRID_STRIDE(i, n) {
-    if (c.ddpm) {
-      const float mean = ADD(MUL(c.w0, x0[i]), MUL(c.wt, xt[i]));                           // DW:293
-      out[i] = ADD(mean, MUL(c.post_std, nz[i]));                                           // DW:297
-    } else {
-      const float et = DIV(SUB(xt[i], MUL(c.sqrt_at, x0[i])), c.sqrt_1m_at);                // DW:299
-      out[i] = ADD(ADD(MUL(c.sqrt_at_next, x0[i]), MUL(c.c2, et)), MUL(c.c1, nz[i]));       // DW:302
-    }
-  }
+  GRID_STRIDE(i, n) out[i] = pixel_posterior_f(x0[i], xt[i], nz[i], c);
 }
 __global__ void pixel_compute_eps_kernel(const float* __restrict__ xt, const float* __restrict__ xn, const float* __restrict__ et_,
                                          cdx_pixel_coef c, float* __restrict__ out, int B, int chw, int net_chw) {
   const size_t n = (size_t)B * chw;
   GRID_STRIDE(i, n) {
     const size_t b = i / chw;
-    const float et = et_[b * net_chw + (i - b * chw)];
-    if (c.ddpm) {
-      const float mean = MUL(c.inv_sqrt_1m_bt, SUB(xt[i], MUL(c.weight, et)));             // DW:266
-      out[i] = DIV(SUB(xn[i], mean), c.std_model);                                          // DW:268
-    } else {
-      const float x0_t = DIV(SUB(xt[i], MUL(et, c.sqrt_1m_at)), c.sqrt_at);                 // DW:271
-      out[i] = DIV(SUB(SUB(xn[i], MUL(c.sqrt_at_next, x0_t)), MUL(c.c2, et)), c.c1);        // DW:275
-    }
+    out[i] = pixel_eps_f(xt[i], xn[i], et_[b * net_chw + (i - b * chw)], c);
   }
 }
 __global__ void pixel_step_kernel(const float* __restrict__ xt, const float* __restrict__ et_, const float* __restrict__ eps,
@@ -319,15 +332,20 @@ __global__ void pixel_step_kernel(const float* __restrict__ xt, const float* __r
   const size_t n = (size_t)B * chw;
   GRID_STRIDE(i, n) {
     const size_t b = i / chw;
-    const float et = et_[b * net_chw + (i - b * chw)];
-    const float nz = eps ? eps[i] : 0.f;
-    if (c.ddpm) {
-      const float mean = MUL(c.inv_sqrt_1m_bt, SUB(xt[i], MUL(c.weight, et)));             // DW:204
-      out[i] = ADD(mean, MUL(MUL(c.mask, c.std_model), nz));                                // DW:208
-    } else {
-      const float x0_t = DIV(SUB(xt[i], MUL(et, c.sqrt_1m_at)), c.sqrt_at);                 // DW:213
-      out[i] = ADD(ADD(MUL(c.sqrt_at_next, x0_t), MUL(c.c2, et)), MUL(c.c1, nz));           // DW:222
-    }
+    out[i] = pixel_step_f(xt[i], et_[b * net_chw + (i - b * chw)], eps ? eps[i] : 0.f, c);
+  }
+}
+// One lock-step iteration of a two-model pixel cycle: the source chain's posterior sample, the noise it recovers from the source
+// U-Net output, and the target chain's update with that noise.  The noise never leaves registers unless z_out asks for it.
+__global__ void pixel_lock_step_kernel(const PixelLockStep a) {
+  GRID_STRIDE(i, a.n) {
+    const size_t b = i / a.chw, r = i - b * a.chw;
+    const float xt = a.xt[i];
+    const float xn = pixel_posterior_f(a.x0[i], xt, a.noise[i], a.cs);                       // sample_xt_next, DW:283-307
+    const float eps = pixel_eps_f(xt, xn, a.et_src[b * a.net_chw_src + r], a.cs);             // compute_eps, DW:230-280
+    a.x_next[i] = xn;
+    if (a.z_out) a.z_out[b * a.z_stride + r] = eps;
+    a.y_next[i] = pixel_step_f(a.y[i], a.et_tgt[b * a.net_chw_tgt + r], eps, a.ct);          // denoising_step_with_eps, DW:114-227
   }
 }
 
@@ -578,6 +596,7 @@ void pixel_step_with_eps(Engine& e, const float* xt, const float* et, const floa
                          int net_chw, cudaStream_t s) {
   LAUNCH1(pixel_step_kernel, (size_t)B * chw, xt, et, eps, c, out, B, chw, net_chw);
 }
+void pixel_lock_step(Engine& e, const PixelLockStep& a, cudaStream_t s) { LAUNCH1(pixel_lock_step_kernel, a.n, a); }
 
 // softmax(q k^T * scale) v through two batched contractions and a row softmax.  Scores live in the arena
 // ([B*heads, Nq, ldS]); the fused tcgen05 flash kernel supersedes this when eligible.

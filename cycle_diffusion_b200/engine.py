@@ -505,6 +505,43 @@ class UNet(Net):
                                      B, Cc, h, w, e.stream))
         return (out, z) if return_z else out
 
+    def cycle_lockstep_pair(self, target, x0, c_src, c_tgt, uc, src_scale, tgt_scale, sched, noise, return_z=False):
+        """cycle_lockstep with this U-Net on the source chain and `target` (a UNet, possibly on another engine of the same device)
+        on the target chain: bit-equal to latent_encode on self followed by latent_decode on target.  Context-free U-Nets pass
+        c_src = c_tgt = uc = None."""
+        e = self.engine
+        x0, noise = _f32c(x0, e.device), _f32c(noise, e.device)
+        c_src, c_tgt, uc = (_f32c(t, e.device) if t is not None else None for t in (c_src, c_tgt, uc))
+        B, Cc, h, w = x0.shape
+        n = sched.refine_steps
+        assert noise.shape == (n + 1, B, Cc, h, w), f'noise shape {tuple(noise.shape)}'
+        assert (c_src is None) == (c_tgt is None) and (c_src is None or c_src.shape == c_tgt.shape)
+        out = e.empty(B, Cc, h, w)
+        z = e.empty(B, n + 1, Cc, h, w) if return_z else None
+        check(lib.cdx_cycle_lockstep_pair(self.h, target.h, _ptr(x0), _ptr(c_src), _ptr(c_tgt), _ptr(uc), c_src.shape[1] if c_src is not None else 0,
+                                          float(src_scale), float(tgt_scale), sched.coef_array(), sched.t_array(), n, _ptr(noise), sched.sqrt_a_T,
+                                          sched.sqrt_1ma_T, _ptr(out), _ptr(z), B, Cc, h, w, e.stream))
+        return (out, z) if return_z else out
+
+    def pixel_cycle_lockstep(self, target, x0, sched, noise, last_noise, return_z=False):
+        """pixel_encode on this U-Net feeding pixel_decode on `target` (a UNet, possibly on another engine of the same device) as one
+        loop: two U-Net calls and one fused kernel per step, no z buffer unless asked for.  x0 [B,C,R,R], noise [es_steps, B,C,R,R]
+        as for pixel_encode, last_noise [1, B,C,R,R] (or None) as for pixel_decode -> target chain result [B,C,R,R] (and
+        z [B, es_steps, C,R,R] when return_z), bit-equal to the two calls."""
+        e = self.engine
+        x0, noise = _f32c(x0, e.device), _f32c(noise, e.device)
+        last_noise = _f32c(last_noise, e.device) if last_noise is not None else None
+        B, Cc, R, _ = x0.shape
+        n = sched.es_steps
+        assert noise.shape == (n, B, Cc, R, R), f'noise shape {tuple(noise.shape)}'
+        assert last_noise is None or last_noise.shape == (1, B, Cc, R, R)
+        out = e.empty(B, Cc, R, R)
+        z = e.empty(B, n, Cc, R, R) if return_z else None
+        t = (C.c_float * n)(*sched.t_loop[:n])
+        check(lib.cdx_pixel_cycle_lockstep(self.h, target.h, _ptr(x0), sched.coef_array(sched.coef[:n]), t, n, _ptr(noise), sched.sqrt_a_T,
+                                           sched.sqrt_1ma_T, _ptr(last_noise), _ptr(out), _ptr(z), B, Cc, R, e.stream))
+        return (out, z) if return_z else out
+
     def pixel_encode(self, x0, sched, noise):
         e = self.engine
         x0, noise = _f32c(x0, e.device), _f32c(noise, e.device)

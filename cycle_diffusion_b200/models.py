@@ -59,8 +59,14 @@ class UnsupervisedTranslation(nn.Module):
             img = self.target_gan_wrapper(z=z, class_label=class_label)
         else:
             assert class_label is None
-            z = self.source_gan_wrapper.encode(image=original_image)
-            img = self.target_gan_wrapper(z=z)
+            src, tgt = self.source_gan_wrapper, self.target_gan_wrapper
+            if getattr(src, 'pair_cycle_applies', None) is not None and src.pair_cycle_applies(tgt):
+                # matching schedules and shapes: the reference's encode -> z -> target (unsupervised_translation.py:48-49) as one
+                # lock-step loop over both models, same result without the z tensor
+                img = src.pair_cycle(tgt, original_image)
+            else:
+                z = src.encode(image=original_image)
+                img = tgt(z=z)
         losses = dict()
         weighted_loss = torch.zeros_like(sample_id).float()
         return (original_image, img), weighted_loss, losses

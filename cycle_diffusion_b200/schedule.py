@@ -136,3 +136,12 @@ class PixelSchedule:
     def coef_array(self, coefs=None):
         coefs = self.coef if coefs is None else coefs
         return (PixelCoef * len(coefs))(*coefs)
+
+    def same_as(self, other):
+        """True when both schedules drive the samplers with the same numbers: sample type, eta, step pairs, betas, log-variances
+        and every per-step scalar."""
+        return (isinstance(other, PixelSchedule) and self.sample_type == other.sample_type and self.eta == other.eta
+                and self.es_steps == other.es_steps and self.pairs == other.pairs and self.t_loop == other.t_loop
+                and torch.equal(self.b, other.b) and np.array_equal(self.logvar, other.logvar)
+                and (self.sqrt_a_T, self.sqrt_1ma_T) == (other.sqrt_a_T, other.sqrt_1ma_T)
+                and bytes(self.coef_array()) == bytes(other.coef_array()))

@@ -439,10 +439,23 @@ class LatentDiffStochasticWrapper(torch.nn.Module):
         n_extra = sched.refine_steps - (eps_list.shape[1] - 1)
         extra = torch.stack([torch.randn(eps_list[:, 0].shape) for _ in range(n_extra)]) if n_extra > 0 else None      # ddim.py:640
         sample = g.unet.latent_decode(eps_list, None, None, 1.0, sched, extra)
+        return self._refine_and_decode(sample)
+
+    def _refine_and_decode(self, sample):
+        g = self.generator
         if self.refine_steps > 0:                                     # refine_eta = 1 (latentdiff_stochastic_wrapper.py:68-77)
             noise = torch.stack([torch.randn(sample.shape) for _ in range(self.refine_steps + 1)])
             sample = g.unet.latent_refine(sample, None, None, 1.0, self.custom_steps, self.refine_steps, noise, g.alphas_cumprod)
         return g.decode_first_stage(sample)
+
+    @staticmethod
+    def _encode_noise(sched, n_rec, shape):
+        noise = torch.zeros((n_rec + 1,) + tuple(shape))
+        noise[0] = torch.randn(shape)
+        for i in range(n_rec):
+            if sched.refine_steps - 1 - i != 0:                        # ddim.py:583-584: the last step returns x0 without a draw
+                noise[1 + i] = torch.randn(shape)
+        return noise
 
     def encode(self, image, class_label=None):
         g, e = self.generator, self.engine
@@ -453,17 +466,41 @@ class LatentDiffStochasticWrapper(torch.nn.Module):
         assert self.eta > 0
         sched = self._sched()
         n_rec = max(0, min(sched.refine_steps, self.white_box_steps - 1))
-        noise = torch.zeros((n_rec + 1,) + tuple(x0.shape))
-        noise[0] = torch.randn(x0.shape)
-        for i in range(n_rec):
-            if sched.refine_steps - 1 - i != 0:                        # ddim.py:583-584: the last step returns x0 without a draw
-                noise[1 + i] = torch.randn(x0.shape)
+        noise = self._encode_noise(sched, n_rec, x0.shape)
         z = g.unet.latent_encode(x0, None, None, 1.0, sched, n_rec, noise).view(bsz, -1)
         assert z.shape[1] == self.latent_dim
         return z
 
     def forward(self, z, class_label=None):
         return self.engine.shift_scale(self.generate(z, class_label), 1.0, 0.5)
+
+    def pair_cycle_applies(self, target):
+        """True when pair_cycle(target, image) computes target(self.encode(image)): the same DDIM schedule (custom_steps, eta,
+        alphas_cumprod) and white_box_steps on both sides, the same resolution and latent shape, no class input, both models on
+        one device, and every step's noise recovered by the encode (white_box_steps - 1 >= the number of DDIM steps)."""
+        if not isinstance(target, LatentDiffStochasticWrapper) or self.enforce_class_input or target.enforce_class_input:
+            return False
+        g, h = self.generator, target.generator
+        return (self.custom_steps == target.custom_steps and self.eta == target.eta and self.white_box_steps == target.white_box_steps
+                and torch.equal(g.alphas_cumprod.float().cpu(), h.alphas_cumprod.float().cpu())
+                and self.resolution == target.resolution and (g.channels, g.image_size) == (h.channels, h.image_size)
+                and self.engine.device == target.engine.device and self.white_box_steps - 1 >= self._sched().refine_steps)
+
+    def pair_cycle(self, target, image):
+        """self.encode(image) followed by target(z), with both DDIM chains advanced in one lock-step loop (cdx_cycle_lockstep_pair:
+        this model's U-Net on the source chain, the target's on the target chain, the recovered noise consumed at once -- no z
+        tensor).  Same random draws in the same order as the two calls (the encode's, then the target's refinement), same result
+        bit for bit.  Called by UnsupervisedTranslation.forward when pair_cycle_applies(target)."""
+        assert self.pair_cycle_applies(target), 'pair_cycle(): schedules / shapes differ (use encode() + target())'
+        g, e = self.generator, self.engine
+        x = e.shift_scale(image, -0.5, 2.0)
+        assert x.shape[2] == x.shape[3] == self.resolution
+        x0 = g.get_first_stage_encoding(g.encode_first_stage(x))
+        assert self.eta > 0
+        sched = self._sched()
+        noise = self._encode_noise(sched, sched.refine_steps, x0.shape)
+        sample = g.unet.cycle_lockstep_pair(target.generator.unet, x0, None, None, None, 1.0, 1.0, sched, noise)
+        return target.engine.shift_scale(target._refine_and_decode(sample), 1.0, 0.5)
 
     @property
     def device(self):
@@ -532,6 +569,10 @@ class DDPMDDIMWrapper(torch.nn.Module):
         shape = eps_list[:, 0].shape
         last = self._randn(shape).unsqueeze(0)       # denoising_step draws once more; the draw is multiplied by 0 (DU:115,131)
         x = self.generator.pixel_decode(eps_list, self.sched, last_noise=last)
+        return self._refine(x)
+
+    def _refine(self, x):
+        bsz, shape = x.shape[0], x.shape
         if self.refine_steps != 0:
             assert self.refine_steps < self.custom_steps
             ref = PixelSchedule(self.sample_type, self.custom_steps, self.es_steps, 1 if self.sample_type == 'ddim' else None, self.t_0)
@@ -553,18 +594,43 @@ class DDPMDDIMWrapper(torch.nn.Module):
             assert class_label is not None
             raise NotImplementedError()
         bsz = image.shape[0]
-        n_rec = self.es_steps - 1
-        if self.rng == 'cuda':
-            noise = torch.randn((n_rec + 1,) + tuple(image.shape), device=e.device)
-        else:
-            noise = torch.stack([torch.randn(image.shape) for _ in range(n_rec + 1)])     # sample_xt, then one per sample_xt_next
+        noise = self._encode_noise(image.shape)
         z = self.generator.pixel_encode(image, self.sched, noise).view(bsz, -1)
         assert z.shape[1] == self.latent_dim
         return z
 
+    def _encode_noise(self, shape):
+        n_rec = self.es_steps - 1
+        if self.rng == 'cuda':
+            return torch.randn((n_rec + 1,) + tuple(shape), device=self.engine.device)
+        return torch.stack([torch.randn(shape) for _ in range(n_rec + 1)])     # sample_xt, then one per sample_xt_next
+
     def forward(self, z, class_label=None):
         img = self.generate(z, class_label)
         return self.engine.shift_scale(img, 1.0, 0.5)
+
+    def pair_cycle_applies(self, target):
+        """True when pair_cycle(target, image) computes target(self.encode(image)): equal PixelSchedules (sample type, eta, steps,
+        betas, variances), the same resolution and channels, no class input, both models on one device."""
+        return (isinstance(target, DDPMDDIMWrapper) and not self.enforce_class_input and not target.enforce_class_input
+                and self.resolution == target.resolution and self.channels == target.channels
+                and self.engine.device == target.engine.device and self.sched.same_as(target.sched))
+
+    def pair_cycle(self, target, image, class_label=None):
+        """self.encode(image) followed by target(z) as one lock-step loop (cdx_pixel_cycle_lockstep): per step one forward of this
+        model's U-Net, one of the target's and one fused kernel; the recovered noise is consumed at once, so the z tensor
+        [B, es_steps*3*R*R] is never materialised.  Random draws are those of the two calls in their order -- this wrapper's encode
+        buffer, then the target's last draw and refinement draws, each with its own `rng` -- and the result is the same bit for bit.
+        The target's refinement (refine_steps, refine_iterations) runs unchanged afterwards.  Called by
+        UnsupervisedTranslation.forward when pair_cycle_applies(target)."""
+        assert self.pair_cycle_applies(target), 'pair_cycle(): schedules / shapes differ (use encode() + target())'
+        e = self.engine
+        x = e.shift_scale(image, -0.5, 2.0)
+        assert x.shape[2] == x.shape[3] == self.resolution
+        noise = self._encode_noise(x.shape)
+        last = target._randn(x.shape).unsqueeze(0)              # denoising_step draws once more; the draw is multiplied by 0 (DU:115,131)
+        y = self.generator.pixel_cycle_lockstep(target.generator, x, self.sched, noise, last)
+        return target.engine.shift_scale(target._refine(y), 1.0, 0.5)
 
     @property
     def device(self):

@@ -271,6 +271,18 @@ int cdx_cycle_lockstep(cdx_net* unet, const float* x0, const float* c_src, const
                        const float* t_host, int n_steps, const float* noise, float sqrt_a_T,
                        float sqrt_1ma_T, float* x_out, float* z_out, int B, int C, int h, int w,
                        void* stream);
+/* cdx_cycle_lockstep for a source and a target network (two unconditional LDMs, latentdiff_stochastic_wrapper.py:253-311: the
+ * DPM-Encoder of one model, ddim.py:450-501, feeding the decode of the other, ddim.py:395-448, as one loop).  Same arguments and
+ * loop as cdx_cycle_lockstep, but each step makes two U-Net calls: the source segments through src_unet and the target segments
+ * through tgt_unet, each chain at the batch it has in cdx_latent_encode / cdx_latent_decode, so the result (and z_out) equals the
+ * two-phase cdx_latent_encode(src_unet) + cdx_latent_decode(tgt_unet) bit for bit.  Context-free U-Nets pass c_src = c_tgt = uc =
+ * NULL and ctx_len = 0.  The two networks may belong to different engines on the same device: both workspaces are sized and both
+ * engines' stream hand-overs are honoured; all work runs on `stream`. */
+int cdx_cycle_lockstep_pair(cdx_net* src_unet, cdx_net* tgt_unet, const float* x0, const float* c_src, const float* c_tgt,
+                            const float* uc, int ctx_len, float src_scale, float tgt_scale, const cdx_ddim_coef* coef,
+                            const float* t_host, int n_steps, const float* noise, float sqrt_a_T,
+                            float sqrt_1ma_T, float* x_out, float* z_out, int B, int C, int h, int w,
+                            void* stream);
 /* The same three loops with PER-SAMPLE guidance scales (device arrays of B floats): the ensemble driver of the text wrappers
  * (SDW:146-165 generate, :189-204 encode -- the reference loops trial x encoder-scale x skip, then x decoder-scale, one chain at a
  * time, recomputing the conditioning and every context K/V projection per member).  Members that share a schedule are batched
@@ -310,6 +322,23 @@ int cdx_pixel_encode(cdx_net* unet, const float* x0, const cdx_pixel_coef* coef,
 int cdx_pixel_decode(cdx_net* unet, const float* z, int n_eps, const cdx_pixel_coef* coef,
                      const float* t_host, int n_steps, const float* last_noise, float* x_out, int B,
                      int C, int R, void* stream);
+
+/* Two-model pixel cycle as one lock-step loop: DDPMDDIMWrapper.encode of src_unet (DW:483-521) feeding DDPMDDIMWrapper.generate's
+ * main loop on tgt_unet (DW:415-429) without a z buffer.  Order of work: x_T = q_sample(x0, noise[0]) with sqrt_a_T / sqrt_1ma_T
+ * taken at index n_steps-1 (the DW:483 quirk); the target chain starts from the same x_T; n_steps-1 iterations, each one src_unet
+ * forward, one tgt_unet forward and ONE fused kernel (sample_xt_next DW:283-307, compute_eps DW:230-280 on the first C channels
+ * of the source output, denoising_step_with_eps DW:114-227 of the target with that noise); then a target-only step for the last
+ * (0, -1) pair with last_noise (multiplied by 0, DU:115,131; may be NULL).
+ *   coef / t_host  host[n_steps] loop order (noisiest first), shared by both chains
+ *   noise          [n_steps, B,C,R,R] dev: noise[0] = x_T draw, noise[1+i] = draw of iteration i (as cdx_pixel_encode)
+ *   x_out          [B,C,R,R] target chain result (before shift / scale)
+ *   z_out          optional [B, n_steps, C,R,R]: the recovered noise, bit-equal to cdx_pixel_encode's z
+ * Each chain runs at batch B on its own network, so x_out equals cdx_pixel_encode(src_unet) + cdx_pixel_decode(tgt_unet) bit for
+ * bit.  The networks may belong to different engines on the same device (both workspaces sized, both stream hand-overs honoured);
+ * all work runs on `stream`. */
+int cdx_pixel_cycle_lockstep(cdx_net* src_unet, cdx_net* tgt_unet, const float* x0, const cdx_pixel_coef* coef,
+                             const float* t_host, int n_steps, const float* noise, float sqrt_a_T, float sqrt_1ma_T,
+                             const float* last_noise, float* x_out, float* z_out, int B, int C, int R, void* stream);
 
 /* ---------------------------------------------------------------- unit-test hooks ----------- */
 /* Individual ops exported for per-op parity tests (tests/test_ops_gpu.py, tests/test_gemm_epilogue_gpu.py).
